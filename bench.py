@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on synthetic Llama-70B-shape matrices.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the workload `w4a16_gemv_llama70b`: the W4A16 (uint4, group 128, GPTQ-style
 quantized zeros, interleaved storage) GEMV at M=1 for the Llama-2-70B linear shapes BASELINE.json configs[1] names
@@ -18,6 +18,10 @@ strong scaling, max-over-ranks device time.
 --impl reference times the reference's only CPU implementation of this path -- the torch dequantise+matmul reference
 program of its tests (testing/python/operators/test_general_matmul_ops_backend_tl.py:227-273), restated in
 oracle/bitblas_oracle.py -- on the host cores, on a bounded row sample of the SAME four shapes.
+
+--dump-outputs DIR writes the four [1, N] outputs of the last timed GEMV step as DIR/gemv_N<N>_K<K>.npy (float32, exact for
+the fp16 results).  Every input is generated from fixed seeds, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -275,6 +279,16 @@ def oracle_gate(bitblas, dev):
     return {"shape_NK": [N, K], "features_checked": ncheck, "criterion": "normwise <= 1e-2 and elementwise rtol=atol=1e-2, 0 mismatches", **report}
 
 
+def dump_outputs(dirname, arrays, limit=64 << 20):
+    """each tensor as <dirname>/<name>.npy in float32"""
+    import numpy as np
+    host = {name: t.float().cpu().numpy() for name, t in arrays.items()}
+    assert sum(a.nbytes for a in host.values()) <= limit, "outputs to dump exceed 64 MB"
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def timed(fn, steps, warmup, barrier=None):
     for _ in range(warmup):
         fn()
@@ -374,12 +388,18 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--skip-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--only", default="", help="comma list of sections to run: gemm,llama,w2a8,formats,e2e (default all; the GEMV step always runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed GEMV step as DIR/<name>.npy (float32; single GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.impl == "reference":
         return run_reference(args)
 
     import torch.distributed as dist
     rank, world, local = dist_env()
+    if args.dump_outputs and world > 1:
+        ap.error("--dump-outputs needs a single-GPU run")
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         os.environ.setdefault("NCCL_DEBUG", "WARN")  # keep NCCL's version banner off stdout: rank 0 prints ONE JSON line
@@ -494,7 +514,7 @@ def main():
         for i, (N, K) in enumerate(GEMV_SHAPES):
             if c == 0:
                 op, prm = make_linear(bitblas, N // world, K, dev, seed=i)
-                A = (torch.rand((1, K), device=dev) - 0.5).half()
+                A = (torch.rand((1, K), generator=torch.Generator(device=dev).manual_seed(100 + i), device=dev) - 0.5).half()
                 out = torch.empty((1, N // world), dtype=torch.float16, device=dev)
             else:
                 op, prm0, A, out = sets[0][i][:4]
@@ -593,6 +613,8 @@ def main():
     torch.cuda.synchronize()
     barrier()
     ms_step = ev0.elapsed_time(ev1) / args.steps
+    if args.dump_outputs:   # every parameter set writes the same `out` tensors: they hold the last timed step's results
+        dump_outputs(args.dump_outputs, {f"gemv_N{N}_K{K}": out for op, prm, A, out, N, K in ops})
     # kernels of this library launched inside the timed region (replayed graph launches are not seen by the library's counter)
     launches = (launches_per_step * args.steps) if step_graphs is not None else (lib.bb_launch_count() - launches0)
     ms_step = max_over_ranks(ms_step)

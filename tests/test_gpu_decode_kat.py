@@ -1,7 +1,8 @@
 """GPU known-answer tests for the in-register LOP3 decode (bb_debug_decode), the analogue of the reference's
 gtest DecodeTest.* suite (testing/cpp/lop3_type_conversion/lowprecision_to_float16.cu:51-101, lowprecision_to_int8.cu):
 values -> compress -> interleave -> device decode -> exact equality.  When oracle/_ref is present the same packed
-words are also decoded by the REFERENCE's device functions (oracle/ref_shim.cu) and compared bit for bit."""
+words are also decoded by the REFERENCE's device functions (oracle/ref_shim.cu) and compared bit for bit; without it the
+tests that compare with the reference check the product against what those functions return, stated in closed form."""
 import ctypes
 import os
 
@@ -57,41 +58,43 @@ def test_decode_to_int8_exact(bits, signed):
     assert np.array_equal(out.cpu().numpy().astype(np.int32), expect)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 @pytest.mark.parametrize("bits,kind_ref", [(4, 0), (2, 2)])
 def test_decode_matches_reference_device_functions(bits, kind_ref):
-    """unsigned decode vs decode_i4u_to_f16 / decode_i2u_to_f16 of fast_decoding.hpp run on this GPU."""
+    """unsigned decode vs decode_i4u_to_f16 / decode_i2u_to_f16 of fast_decoding.hpp run on this GPU; they return the fields."""
     lib = _lib.load()
     _lib.ensure_init(0)
-    ref = ctypes.CDLL(REF_SO)
-    ref.ref_decode_f16.argtypes = [ctypes.c_int] + [ctypes.c_void_p] * 2 + [ctypes.c_int] + [ctypes.c_void_p] * 4
     rng = np.random.RandomState(5)
     vals = rng.randint(0, 2**bits, size=(1, 8192)).astype(np.int8)
     dev = _pack(vals, bits, "float16")
     mine = torch.empty(8192, dtype=torch.float16, device="cuda")
-    theirs = torch.empty(8192, dtype=torch.float16, device="cuda")
     _lib.check(lib.bb_debug_decode(0, bits, 0, _lib.BB_LAYOUT_INTERLEAVED_16, dev.data_ptr(), mine.data_ptr(), dev.numel() // 4, 0))
-    assert ref.ref_decode_f16(kind_ref, dev.data_ptr(), theirs.data_ptr(), 8192 // 8, None, None, None, None) == 0
     torch.cuda.synchronize()
-    assert torch.equal(mine, theirs)
-    assert np.array_equal(theirs.cpu().numpy().astype(np.int32), vals.reshape(-1))
+    assert np.array_equal(mine.cpu().numpy().astype(np.int32), vals.reshape(-1))
+    ref = _ref_lib()
+    if ref is not None:
+        theirs = torch.empty(8192, dtype=torch.float16, device="cuda")
+        assert ref.ref_decode_f16(kind_ref, dev.data_ptr(), theirs.data_ptr(), 8192 // 8, None, None, None, None) == 0
+        torch.cuda.synchronize()
+        assert torch.equal(mine, theirs)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 def test_int8_decode_matches_reference_device_functions():
+    """unsigned 2-bit decode to int8 vs decode_i2u_to_i8s of fast_decoding.hpp run on this GPU; it returns the fields."""
     lib = _lib.load()
     _lib.ensure_init(0)
-    ref = ctypes.CDLL(REF_SO)
-    ref.ref_decode_i8.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
     rng = np.random.RandomState(6)
     vals = rng.randint(0, 4, size=(1, 4096)).astype(np.int8)
     dev = _pack(vals, 2, "int8")
     mine = torch.empty(4096, dtype=torch.int8, device="cuda")
-    theirs = torch.empty(4096, dtype=torch.int8, device="cuda")
     _lib.check(lib.bb_debug_decode(2, 2, 0, _lib.BB_LAYOUT_INTERLEAVED_8, dev.data_ptr(), mine.data_ptr(), dev.numel() // 4, 0))
-    assert ref.ref_decode_i8(2, dev.data_ptr(), theirs.data_ptr(), 4096 // 16, None) == 0
     torch.cuda.synchronize()
-    assert torch.equal(mine, theirs)
+    assert np.array_equal(mine.cpu().numpy(), vals.reshape(-1))
+    ref = _ref_lib()
+    if ref is not None:
+        theirs = torch.empty(4096, dtype=torch.int8, device="cuda")
+        assert ref.ref_decode_i8(2, dev.data_ptr(), theirs.data_ptr(), 4096 // 16, None) == 0
+        torch.cuda.synchronize()
+        assert torch.equal(mine, theirs)
 
 
 @pytest.mark.parametrize("bits", [4, 2, 1])
@@ -113,13 +116,15 @@ REF_I8 = dict(I4U=0, I4S=1, I2U=2, I2S=3, I1U=4, I1S=5)
 
 
 def _ref_lib():
+    """the reference's decode functions (oracle/build_ref.py), or None where they are not built"""
+    if not os.path.exists(REF_SO):
+        return None
     ref = ctypes.CDLL(REF_SO)
     ref.ref_decode_f16.argtypes = [ctypes.c_int] + [ctypes.c_void_p] * 2 + [ctypes.c_int] + [ctypes.c_void_p] * 4
     ref.ref_decode_i8.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
     return ref
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 @pytest.mark.parametrize("bits,kind", [(4, "I4S"), (2, "I2S")])
 def test_signed_decode_vs_reference_device_functions(bits, kind):
     """decode_i{4,2}s_to_f16: the reference's C++ harness subtracts 2^(b-1) - 1 (fast_decoding.hpp:17, MEDIAN 0x6407 / 0x6401)
@@ -127,19 +132,20 @@ def test_signed_decode_vs_reference_device_functions(bits, kind):
     the two decodes must differ by exactly one everywhere (SURVEY.md 8c)."""
     lib = _lib.load()
     _lib.ensure_init(0)
-    ref = _ref_lib()
     vals = np.random.RandomState(11).randint(0, 2**bits, size=(1, 8192)).astype(np.int8)
     dev = _pack(vals, bits, "float16")
     mine = torch.empty(8192, dtype=torch.float16, device="cuda")
-    theirs = torch.empty(8192, dtype=torch.float16, device="cuda")
     _lib.check(lib.bb_debug_decode(0, bits, 1, _lib.BB_LAYOUT_INTERLEAVED_16, dev.data_ptr(), mine.data_ptr(), dev.numel() // 4, 0))
-    assert ref.ref_decode_f16(REF_F16[kind], dev.data_ptr(), theirs.data_ptr(), 8192 // 8, None, None, None, None) == 0
     torch.cuda.synchronize()
-    assert torch.equal(mine + 1, theirs)
     assert np.array_equal(mine.cpu().numpy().astype(np.int32), vals.reshape(-1).astype(np.int32) - 2 ** (bits - 1))
+    ref = _ref_lib()
+    if ref is not None:
+        theirs = torch.empty(8192, dtype=torch.float16, device="cuda")
+        assert ref.ref_decode_f16(REF_F16[kind], dev.data_ptr(), theirs.data_ptr(), 8192 // 8, None, None, None, None) == 0
+        torch.cuda.synchronize()
+        assert torch.equal(mine + 1, theirs)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 @pytest.mark.parametrize("kind,bits,mode", [
     ("I4U_SCALE", 4, 1), ("I4U_ZEROS_ORIGINAL", 4, 2), ("I4U_ZEROS_RESCALE", 4, 3), ("I4U_ZEROS_QUANTIZED", 4, 4),
     ("I2U_SCALE", 2, 1), ("I2U_ZEROS_ORIGINAL", 2, 2), ("I2U_ZEROS_RESCALE", 2, 3)])
@@ -149,7 +155,6 @@ def test_dequant_arithmetic_vs_reference_device_functions(kind, bits, mode):
     non-trivial fp16 scales and non-integer fp16 zero points (one per group of 8 outputs, as in the reference KATs)."""
     lib = _lib.load()
     _lib.ensure_init(0)
-    ref = _ref_lib()
     rng = np.random.RandomState(12)
     n = 16384
     vals = rng.randint(0, 2**bits, size=(1, n)).astype(np.int8)
@@ -162,13 +167,16 @@ def test_dequant_arithmetic_vs_reference_device_functions(kind, bits, mode):
     zeros = torch.from_numpy(zeros_np).cuda()
     qz = torch.from_numpy(rng.randint(0, 2**bits, size=g).astype(np.int32)).cuda()
     mine = torch.empty(n, dtype=torch.float16, device="cuda")
-    theirs = torch.empty(n, dtype=torch.float16, device="cuda")
     _lib.check(lib.bb_debug_dequant(0, bits, 0, _lib.BB_LAYOUT_INTERLEAVED_16, mode, dev.data_ptr(), scale.data_ptr(),
                                     zeros.data_ptr(), qz.data_ptr(), mine.data_ptr(), dev.numel() // 4, 0))
-    assert ref.ref_decode_f16(REF_F16[kind], dev.data_ptr(), theirs.data_ptr(), g, scale.data_ptr(),
-                              zeros.data_ptr() if mode in (2, 3) else None, qz.data_ptr() if mode == 4 else None, None) == 0
     torch.cuda.synchronize()
-    assert torch.equal(mine, theirs), (mine[:16], theirs[:16])
+    ref = _ref_lib()
+    if ref is not None:
+        theirs = torch.empty(n, dtype=torch.float16, device="cuda")
+        assert ref.ref_decode_f16(REF_F16[kind], dev.data_ptr(), theirs.data_ptr(), g, scale.data_ptr(),
+                                  zeros.data_ptr() if mode in (2, 3) else None, qz.data_ptr() if mode == 4 else None, None) == 0
+        torch.cuda.synchronize()
+        assert torch.equal(mine, theirs), (mine[:16], theirs[:16])
     # and the oracle's A_dtype dequantise (the model every parity test is checked against) states the same numbers
     u = torch.from_numpy(vals.reshape(-1).astype(np.float32)).half()
     s8, z8, q8 = (scale.cpu().repeat_interleave(8), zeros.cpu().repeat_interleave(8), qz.cpu().repeat_interleave(8).half())
@@ -177,24 +185,25 @@ def test_dequant_arithmetic_vs_reference_device_functions(kind, bits, mode):
     assert torch.equal(mine.cpu(), expect)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 @pytest.mark.parametrize("kind,bits,signed", [("I4U", 4, 0), ("I4S", 4, 1), ("I2U", 2, 0), ("I2S", 2, 1)])
 def test_int8_decode_matrix_vs_reference_device_functions(kind, bits, signed):
     """lowprecision_to_int8.cu DecodeTest.{U,}Int{4,2}ToINT8.  Signed: the reference harness subtracts 2^(b-1) - 1
     (decode_i4s_to_i8s: 7, lop3.py:1016 -- SURVEY.md 8c defect (iii)); the Python product and this library subtract 2^(b-1)."""
     lib = _lib.load()
     _lib.ensure_init(0)
-    ref = _ref_lib()
     vals = np.random.RandomState(13).randint(0, 2**bits, size=(1, 8192)).astype(np.int8)
     dev = _pack(vals, bits, "int8")
     mine = torch.empty(8192, dtype=torch.int8, device="cuda")
-    theirs = torch.empty(8192, dtype=torch.int8, device="cuda")
     _lib.check(lib.bb_debug_decode(2, bits, signed, _lib.BB_LAYOUT_INTERLEAVED_8, dev.data_ptr(), mine.data_ptr(), dev.numel() // 4, 0))
-    assert ref.ref_decode_i8(REF_I8[kind], dev.data_ptr(), theirs.data_ptr(), 8192 // 16, None) == 0
     torch.cuda.synchronize()
     assert np.array_equal(mine.cpu().numpy().astype(np.int32), vals.reshape(-1).astype(np.int32) - (2 ** (bits - 1) if signed else 0))
-    delta = (theirs.cpu().to(torch.int32) - mine.cpu().to(torch.int32))
-    assert (delta == (1 if signed else 0)).all(), delta.unique()
+    ref = _ref_lib()
+    if ref is not None:
+        theirs = torch.empty(8192, dtype=torch.int8, device="cuda")
+        assert ref.ref_decode_i8(REF_I8[kind], dev.data_ptr(), theirs.data_ptr(), 8192 // 16, None) == 0
+        torch.cuda.synchronize()
+        delta = (theirs.cpu().to(torch.int32) - mine.cpu().to(torch.int32))
+        assert (delta == (1 if signed else 0)).all(), delta.unique()
 
 
 @pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
